@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            (N>1: launched under torchrun, one rank per GPU)
     python bench.py --impl reference --gpus N --steps K --warmup W
+    python bench.py ... --dump-outputs DIR       (also write what the last timed step computed as DIR/<name>.npy)
 
 Headline workload (BASELINE.json configs[1], "C2"): batch keccak256 of 10M 32-byte keys per GPU — the
 AccountHashing / StorageHashing inner loop.  One step = one pass over the batch.
@@ -44,6 +45,9 @@ C3_ACCOUNTS = 1_000_000
 C3_SLOTS = 16
 METRIC = "keccak256_digests_per_sec"
 UNIT = "digests/s"
+DUMP_SEED = 20240917
+DUMP_ROWS = 131_072        # sampled digest rows: 131072 x 32 float32 = 16 MB
+DUMP_MAX_BYTES = 64 << 20
 
 
 def effective_cpus() -> int:
@@ -91,6 +95,35 @@ def c2_config(n_keys: int, world: int) -> dict:
     return {"workload": "C2: batch keccak256 of 10M 32-byte keys per GPU (AccountHashing/StorageHashing inner loop)",
             "keys_per_gpu": n_keys, "msg_len": 32, "parallelism": f"keys sharded over {world} GPU(s), no collective",
             "l2": "input 320 MB + output 320 MB per step exceed the 126 MB L2; no flush needed"}
+
+
+# ------------------------------------------------------------------------------------------------ --dump-outputs
+def dump_rows(n: int) -> np.ndarray:
+    """Ascending digest rows --dump-outputs writes: all of them up to DUMP_ROWS, else a fixed sample seeded by DUMP_SEED,
+    so that two builds run with the same arguments write the same rows."""
+    if n <= DUMP_ROWS:
+        return np.arange(n, dtype=np.int64)
+    return np.sort(np.random.default_rng(DUMP_SEED).choice(n, DUMP_ROWS, replace=False))
+
+
+def keccak_dump(digests: np.ndarray, rows: np.ndarray) -> dict:
+    """digests: uint8 [len(rows), 32], the digests of `rows` of the batch."""
+    return {"keccak_digests": digests.astype(np.float32), "keccak_digest_rows": rows.astype(np.float64)}
+
+
+def root_dump(root_hex: str) -> np.ndarray:
+    return np.frombuffer(bytes.fromhex(root_hex), np.uint8).astype(np.float32)
+
+
+def write_dumps(out_dir: str, arrays: dict) -> None:
+    """Writes every array as out_dir/<name>.npy: bytes as float32, row indices as float64 (exact below 2^53)."""
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_MAX_BYTES:
+        raise SystemExit(f"--dump-outputs: {total} bytes exceed the {DUMP_MAX_BYTES}-byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 # ------------------------------------------------------------------------------------------------ synthetic data
@@ -313,8 +346,11 @@ def run_reference(args, rank, world):
         oracle.keccak256_fixed(keys, threads=cores)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        oracle.keccak256_fixed(keys, threads=cores)
+        out = oracle.keccak256_fixed(keys, threads=cores)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        rows = dump_rows(n)
+        write_dumps(args.dump_outputs, keccak_dump(out[rows], rows))
     val = n * args.steps / dt
     sample = f"each step hashes all {n} 32-byte keys on {cores} host threads (scalar C keccak, chunks of 100)"
     simd_val = None
@@ -363,7 +399,12 @@ def main():
     ap.add_argument("--skip-cpu", action="store_true")
     ap.add_argument("--skip-dynamic", action="store_true", help="skip the in-place block-update legs (dynamic resident trie / "
                     "state: tools/dtrie_bench.py, tools/dstate_bench.py, each in its own process) and the f2/f3/f4 throughput legs")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last step computed as "
+                    "DIR/<name>.npy (float32/float64, rank 0): a seeded sample of the keccak digests with its row indices, "
+                    "and the roots of the state-root legs that ran")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
 
     rank, world, local_rank = env_int("RANK", 0), env_int("WORLD_SIZE", 1), env_int("LOCAL_RANK", 0)
@@ -447,6 +488,10 @@ def main():
     got = d_out.view(n, 32)[idx].cpu().numpy()
     exp = oracle.keccak256_fixed(d_keys.view(n, 32)[idx].cpu().numpy())
     parity_ok = bool((got == exp).all())
+    dumps = {}
+    if args.dump_outputs and rank == 0:
+        rows = dump_rows(n)
+        dumps.update(keccak_dump(d_out.view(n, 32)[torch.from_numpy(rows).to(dev)].cpu().numpy(), rows))
 
     # ---------------------------------------------------------------- C2 e2e: host buffers through the C ABI
     h_in = eng.pinned_empty((n, 32))
@@ -513,6 +558,12 @@ def main():
         }
         if dynamic is not None:
             line["dynamic"] = dynamic
+        if args.dump_outputs:
+            for name, leg, key in (("state_root", state_root, "root"), ("mainnet_shape_root", c4, "root"),
+                                   ("incremental_root", incremental, "root_after")):
+                if leg and leg.get(key):
+                    dumps[name] = root_dump(leg[key])
+            write_dumps(args.dump_outputs, dumps)
         emit(line)
     if comm is not None:
         comm.close()
