@@ -84,9 +84,7 @@ extern "C" B200_API b200_ctx *b200_create(int32_t device_ordinal) {
     if ((e = cudaEventCreate(&c->ev0)) != cudaSuccess) return bail(e);
     if ((e = cudaEventCreate(&c->ev1)) != cudaSuccess) return bail(e);
     if ((e = cudaMallocHost(&c->pinned_small, 4096)) != cudaSuccess) return bail(e);
-    if ((e = cudaMalloc(&c->small.p, SM_WORDS * 4)) != cudaSuccess) return bail(e);
-    c->small.cap = SM_WORDS * 4;
-    c->dev_bytes += c->small.cap;
+    if ((e = c->small.grow(SM_WORDS * 4, SM_WORDS * 4, c->stream)) != cudaSuccess) return bail(e);
     if ((e = cudaMemset(c->small.p, 0, SM_WORDS * 4)) != cudaSuccess) return bail(e);
     c->phase_timing = getenv("B200_PHASE_TIMING") != nullptr;
     g_create_status = B200_OK;
@@ -97,16 +95,6 @@ extern "C" B200_API void b200_destroy(b200_ctx *c) {
     if (!c) return;
     cudaSetDevice(c->device);
     cudaDeviceSynchronize();
-    DevBuf *bufs[] = {&c->Lp, &c->nibs, &c->leaf_ref, &c->leaf_meta, &c->S, &c->E, &c->iota, &c->depth_sorted,
-                      &c->gap_sorted, &c->head, &c->node_start, &c->node_ref, &c->node_meta,
-                      &c->node_l, &c->node_r, &c->node_masks, &c->cub_temp, &c->small, &c->sroots, &c->buckets,
-                      &c->upd_flags, &c->upd_nh, &c->upd_ids, &c->upd_prefix, &c->upd_key, &c->upd_key2, &c->upd_ids2, &c->in_a, &c->in_b, &c->in_c,
-                      &c->in_d, &c->in_e, &c->out_a, &c->chunk_in[0], &c->chunk_in[1], &c->chunk_in[2], &c->chunk_out[0],
-                      &c->chunk_out[1], &c->chunk_out[2], &c->sort_ka, &c->sort_kb, &c->sort_ia, &c->sort_flag, &c->sort_perm,
-                      &c->sort_out, &c->sort_aux[0], &c->sort_aux[1], &c->sort_aux[2], &c->sort_aux[3], &c->node_key, &c->node_key2, &c->node_ids, &c->node_order, &c->ord_keys, &c->ord_knib,
-                      &c->ord_item, &c->ord_sched, &c->ord_sched2, &c->ord_pos, &c->ord_order};
-    for (DevBuf *b : bufs)
-        if (b->p) cudaFree(b->p);
     if (c->pinned_small) cudaFreeHost(c->pinned_small);
     if (c->ev_fork) cudaEventDestroy(c->ev_fork);
     if (c->ev_join) cudaEventDestroy(c->ev_join);
@@ -119,7 +107,7 @@ extern "C" B200_API void b200_destroy(b200_ctx *c) {
     for (int i = 0; i < 3; i++)
         if (c->copy_streams[i]) cudaStreamDestroy(c->copy_streams[i]);
     if (c->own_stream) cudaStreamDestroy(c->own_stream);
-    delete c;
+    delete c;  // frees the scratch buffers
 }
 
 extern "C" B200_API const char *b200_last_error(const b200_ctx *c) {
